@@ -2,6 +2,7 @@
 """bench.py -- fpng hot-path benchmark (encode MP/s on synthetic batches) for the B200-native implementation.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c1] [--kind g1|g0|g2]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the encode hot path over one batch of synthetic images (device-resident for `value`,
 host-resident pinned buffers through the C ABI for `e2e`).  Prints ONE JSON line on rank 0.  See DESIGN.md section
@@ -84,6 +85,40 @@ def make_device_batch(wl, kind: str, n: int, device, first_index: int = 0):
             img = img + noises[i % N_UNIQUE_NOISE]
         batch[k] = (img & 255).to(torch.uint8)
     return batch
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dump_dir: str, out, sizes):
+    """Writes what the last timed encode step returned to its caller, as float arrays a later build's dump can be compared with:
+    sizes.npy (float64, every file's size) and files.npy (float32 [k, m]: the bytes of the k files files_index.npy names, chosen
+    with a fixed seed, -1 past a file's end).  A file longer than its share of the 64 MB is sampled at positions drawn with a fixed
+    seed, always including its last 16 bytes (Adler-32, IDAT CRC-32 and IEND depend on every byte before them); files_positions.npy
+    (float64) says where."""
+    n = out.shape[0]
+    sz = sizes.cpu().numpy().astype(np.int64) & 0xFFFFFFFF
+    rs = np.random.RandomState(0)
+    pick = np.sort(rs.choice(n, size=min(n, 4), replace=False))
+    cap = (DUMP_BYTES - (1 << 20)) // (12 * len(pick))       # 4 bytes in files.npy + 8 in files_positions.npy per sampled byte
+    rows, pos = [], []
+    for i in pick:
+        size = int(sz[i])
+        p = np.arange(size) if size <= cap else \
+            np.union1d(np.sort(rs.choice(size - 16, size=cap - 16, replace=False)), np.arange(size - 16, size))
+        rows.append(out[i].cpu().numpy()[p])
+        pos.append(p)
+    m = max(len(p) for p in pos)
+    files = np.full((len(pick), m), -1, np.float32)
+    where = np.full((len(pick), m), -1, np.float64)
+    for k, (r, p) in enumerate(zip(rows, pos)):
+        files[k, :len(r)] = r
+        where[k, :len(p)] = p
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, "sizes.npy"), sz.astype(np.float64))
+    np.save(os.path.join(dump_dir, "files.npy"), files)
+    np.save(os.path.join(dump_dir, "files_positions.npy"), where)
+    np.save(os.path.join(dump_dir, "files_index.npy"), pick.astype(np.float64))
 
 
 class ClockSampler:
@@ -340,6 +375,8 @@ def run_ours(args, wl):
     if world > 1:
         dist.barrier()
     clocks = sampler.stop(wall0, wall1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, sizes)
     launches = fpng_b200.launch_count() - launches0
     ms = e0.elapsed_time(e1)
     prof = (C.c_float * 9)()
@@ -685,7 +722,13 @@ def main():
     ap.add_argument("--encoder", default="default", choices=["default", "two_kernel", "two_kernel_serial", "two_kernel_file_crc", "fused"],
                     help="default: the library's choice; two_kernel: scan+pack with the chunked CRC overlap; two_kernel_serial: scan+pack, serial; two_kernel_file_crc: scan+pack, IDAT CRC by the file-reading kernel instead of the pack kernel; fused: single-pass encoder")
     ap.add_argument("--own-files", action="store_true", help="decode leg: use the GPU-written files instead of reference-written ones")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the encoded files of the last step (sizes and a fixed sample of files) as .npy to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU encoder's outputs; --impl reference has none")
     args.auto_workload = args.workload == "auto"
     if args.workload == "auto":
         args.workload = "c2" if max(args.gpus, int(os.environ.get("WORLD_SIZE", "1"))) <= 1 else "c3"

@@ -37,7 +37,8 @@ def build(force: bool = False) -> None:
         (not os.path.exists(REF_SO)) or os.path.getmtime(REF_SO) < os.path.getmtime(os.path.join(HERE, "ref_shim.cpp"))
         or (not os.path.exists(REF_TRAIN_SO)) or os.path.getmtime(REF_TRAIN_SO) < os.path.getmtime(os.path.join(HERE, "ref_train_shim.cpp"))
         or (not os.path.exists(REF_PATCH_SO)) or os.path.getmtime(REF_PATCH_SO) < os.path.getmtime(os.path.join(HERE, "ref_patch_shim.cpp"))
-        or (not os.path.exists(VERIFIERS_SO)) or os.path.getmtime(VERIFIERS_SO) < os.path.getmtime(os.path.join(HERE, "verifiers_shim.cpp")))
+        or (not os.path.exists(VERIFIERS_SO)) or os.path.getmtime(VERIFIERS_SO) < os.path.getmtime(os.path.join(HERE, "verifiers_shim.cpp"))
+        or not os.path.exists(os.path.join(HERE, "_ref", "fpng_test_train")))
     if force or stale or ref_stale:
         subprocess.check_call(["make", "-s", "-f", os.path.join(HERE, "Makefile"), "all"], cwd=HERE)
 

@@ -1,4 +1,5 @@
-"""Tests against the REAL reference harness (fpng_test compiled from /root/reference/src where it lies, test-only, into oracle/_ref/).
+"""Tests against the REAL reference harness (fpng_test compiled from the reference sources, test-only, into oracle/_ref/; its
+recorded output, tests/reference_answers.py, where the reference is absent).
 
 1. tools/train_tables.py (the `fpng_test -t` counterpart) against the REAL harness: the unmodified reference's fpng_test is compiled
 with its own FPNG_TRAIN_HUFFMAN_TABLES=1 switch (into oracle/_ref/, test-only) and run on a listing of PNG files; the driver -- with
@@ -10,7 +11,6 @@ reference trainer by tests/test_training_gpu.py.
 2. BASELINE config 1 through the harness's own plumbing (see test_config1_through_the_real_harness_plumbing)."""
 import io
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -19,29 +19,24 @@ import pytest
 import imagegen
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SRC = "/root/reference/src"
 HARNESS = os.path.join(ROOT, "oracle", "_ref", "fpng_test_train")
 
 
-@pytest.fixture(scope="module")
-def harness():
-    if not os.path.exists(HARNESS):
-        if not os.path.exists(os.path.join(REF_SRC, "fpng_test.cpp")):
-            pytest.skip("reference tree not present and no prebuilt harness")
-        os.makedirs(os.path.dirname(HARNESS), exist_ok=True)
-        subprocess.check_call(["g++", "-O1", "-std=c++11", "-fno-strict-aliasing", "-msse4.1", "-mpclmul", "-DFPNG_NO_SSE=0",
-                               "-DFPNG_TRAIN_HUFFMAN_TABLES=1", "-w", "-I" + REF_SRC] +
-                              [os.path.join(REF_SRC, f) for f in ("fpng.cpp", "fpng_test.cpp", "lodepng.cpp", "pvpngreader.cpp")] +
-                              ["-o", HARNESS, "-lm", "-lpthread"])
-    return HARNESS
+@pytest.fixture
+def harness(request):
+    """fpng_test built in training mode (same encoder output) by oracle/Makefile, as recorded (tests/reference_answers.py)"""
+    import reference_answers as ra
+    real = HARNESS if ra.recording(lambda: os.path.exists(HARNESS)) else None
+    calls = ra.Calls(ra.answer_key(request, "harness"), real)
+    yield ra.RecordedHarness(calls)
+    calls.finish()
 
 
 class ReferenceTrainerBackend:
     """stands in for tools/train_tables.py GpuBackend (same three calls) on a box without a device"""
 
-    def __init__(self):
-        from oracle.pyoracle import RefTrainer, Ref
-        self.t, self.ref = RefTrainer(), Ref()
+    def __init__(self, trainer, ref):
+        self.t, self.ref = trainer, ref
 
     def accumulate(self, img, counts):
         h, w, c = img.shape
@@ -78,11 +73,11 @@ def _write_pngs(tmp, oracle):
     return listing
 
 
-def test_training_driver_prints_what_the_real_harness_prints(tmp_path, oracle, harness):
+def test_training_driver_prints_what_the_real_harness_prints(tmp_path, oracle, harness, ref_trainer, ref):
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     import train_tables
     listing = _write_pngs(str(tmp_path), oracle)
-    real = subprocess.run([harness, "-t", "@" + listing], capture_output=True, text=True)
+    real, _ = harness.run(["-t", "@" + listing], cwd=tmp_path)
     assert real.returncode == 0, real.stderr
     # the harness prints a banner / SSE line first; compare from the listing line on
     real_lines = real.stdout.splitlines()
@@ -90,7 +85,7 @@ def test_training_driver_prints_what_the_real_harness_prints(tmp_path, oracle, h
     buf = io.StringIO()
     files = train_tables.load_listing("@" + listing)
     assert len(files) == 8
-    tables = train_tables.train(files, ReferenceTrainerBackend(), out=buf)
+    tables = train_tables.train(files, ReferenceTrainerBackend(ref_trainer, ref), out=buf)
     mine = [real_lines[start]] + buf.getvalue().splitlines()
     assert mine == real_lines[start:], "\n".join(f"{a!r}\n{b!r}" for a, b in zip(mine, real_lines[start:]) if a != b)
     assert "Total alpha files: 3" in mine and "Total opaque files: 4" in mine and "Total failed loading: 1" in mine
@@ -112,12 +107,11 @@ def test_config1_through_the_real_harness_plumbing(tmp_path, oracle, harness, op
     assert img.shape == (h, w, c) and (img[:, :, 3] < 255).any()
     src = tmp_path / "c1_g0.png"
     Image.fromarray(img, "RGBA").save(src)
-    r = subprocess.run([harness, *opts, str(src)], capture_output=True, text=True, cwd=tmp_path)        # fpng.png is written without -c
+    r, out = harness.run([*opts, str(src)], cwd=tmp_path)        # fpng.png is written without -c
     assert r.returncode == 0, r.stdout[-500:] + r.stderr[-500:]
     assert "Has Alpha: 1" in r.stdout
-    out = (tmp_path / "fpng.png").read_bytes()
     assert out == oracle.encode(img, w, h, c, flags)
-    r = subprocess.run([harness, "-c", *opts, str(src)], capture_output=True, text=True, cwd=tmp_path)
+    r, _ = harness.run(["-c", *opts, str(src)], cwd=tmp_path)
     assert r.returncode == 0, r.stdout[-500:] + r.stderr[-500:]
     # CSV row: file, w, h, chans, then {enc s, MB, dec s, enc MP/s, dec MP/s} for qoi, fpng, lodepng, stbi, and pvpng's two
     row = [t.strip() for t in r.stdout.strip().splitlines()[-1].split(",")]

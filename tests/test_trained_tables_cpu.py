@@ -17,16 +17,13 @@ def load_tables():
 
 
 @pytest.mark.parametrize("chans", [3, 4])
-def test_oracle_custom_table_matches_golden_and_patched_reference(oracle, chans):
+def test_oracle_custom_table_matches_golden_and_patched_reference(oracle, ref_patched, chans):
     t = load_tables()[str(chans)]
     prefix = bytes.fromhex(t["prefix"])
     sizes = np.array(t["sizes"], np.uint8)
     assert chans == 3 or t["rule_hits"] > 50            # the fixture makes the rule fire
-    rp = None
-    from oracle.pyoracle import RefPatched
-    if RefPatched.available():
-        rp = RefPatched()
-        assert rp.set_table(chans, prefix, t["bit_buf"], t["bit_buf_size"], t["codes"], t["sizes"])
+    rp = ref_patched
+    assert rp.set_table(chans, prefix, t["bit_buf"], t["bit_buf_size"], t["codes"], t["sizes"])
     try:
         assert oracle.set_static_table(chans, prefix, t["bit_buf"], t["bit_buf_size"])
         got_sizes, got_codes, hb = oracle.static_table(chans)
@@ -37,14 +34,12 @@ def test_oracle_custom_table_matches_golden_and_patched_reference(oracle, chans)
             assert (name, w, h) == (vec["name"], vec["w"], vec["h"])
             png = oracle.encode(img, w, h, chans, 0)
             assert sha(png) == vec["sha256"] and len(png) == vec["size"], name
-            if rp is not None:
-                assert png == rp.encode(img, w, h, chans, 0), name
+            assert png == rp.encode(img, w, h, chans, 0), name
             st, px, *_ = oracle.decode(png, chans)
             assert st == 0 and np.array_equal(px, img.reshape(-1))
     finally:
         oracle.set_static_table(chans)
-        if rp is not None:
-            rp.reset_table(chans)
+        rp.reset_table(chans)
     # restored: shipped table again
     img = imagegen.make("g1", 64, 8, chans, 0)
     assert sha(oracle.encode(img, 64, 8, chans, 0)) == sha(oracle.encode(img, 64, 8, chans, 0))

@@ -12,15 +12,13 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("chans", [3, 4])
-def test_trained_table_byte_parity(gpu, oracle, ref, chans):
+def test_trained_table_byte_parity(gpu, oracle, ref, ref_patched, chans):
     import torch
     t = load_tables()[str(chans)]
     prefix = bytes.fromhex(t["prefix"])
     sizes = np.array(t["sizes"], np.uint8)
-    from oracle.pyoracle import RefPatched
-    rp = RefPatched() if RefPatched.available() else None
-    if rp is not None:
-        assert rp.set_table(chans, prefix, t["bit_buf"], t["bit_buf_size"], t["codes"], t["sizes"])
+    rp = ref_patched
+    assert rp.set_table(chans, prefix, t["bit_buf"], t["bit_buf_size"], t["codes"], t["sizes"])
     assert oracle.set_static_table(chans, prefix, t["bit_buf"], t["bit_buf_size"])
     try:
         gpu.set_static_table(chans, prefix, t["bit_buf"], t["bit_buf_size"])
@@ -29,8 +27,7 @@ def test_trained_table_byte_parity(gpu, oracle, ref, chans):
             assert ok
             assert sha(png) == vec["sha256"], (name, len(png), vec["size"])
             assert png == oracle.encode(img, w, h, chans, 0), name
-            if rp is not None:
-                assert png == rp.encode(img, w, h, chans, 0), name
+            assert png == rp.encode(img, w, h, chans, 0), name
             st, px, *_ = ref.decode(png, chans)                      # the unmodified reference decoder reads the table from the stream
             assert st == 0 and np.array_equal(px, img.reshape(-1))
             st, px, *_ = gpu.fpng_decode_memory(png, chans)
@@ -51,8 +48,7 @@ def test_trained_table_byte_parity(gpu, oracle, ref, chans):
     finally:
         gpu.set_static_table(chans)
         oracle.set_static_table(chans)
-        if rp is not None:
-            rp.reset_table(chans)
+        rp.reset_table(chans)
     im = imagegen.make("g1", 64, 8, chans, 0)
     assert gpu.fpng_encode_image_to_memory(im, 64, 8, chans, 0)[1] == ref.encode(im, 64, 8, chans, 0)
 

@@ -10,27 +10,19 @@ import imagegen
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module")
-def trainer():
-    from oracle.pyoracle import RefTrainer
-    if not RefTrainer.available():
-        pytest.skip("oracle/_ref/libfpng_ref_train.so not available")
-    return RefTrainer()
-
-
 @pytest.mark.parametrize("workload", ["mixed", "noisy"])
 @pytest.mark.parametrize("chans", [3, 4])
-def test_training_matches_reference(gpu, ref, trainer, chans, workload):
+def test_training_matches_reference(gpu, ref, ref_trainer, chans, workload):
     import torch
     w, h, n = 256, 96, 6
     kinds = ["g1", "g0", "runs"] if workload == "mixed" else ["g1"]
     imgs = [imagegen.make(kinds[i % len(kinds)], w, h, chans, i) for i in range(n)]
     dev = torch.from_numpy(np.stack(imgs)).cuda()
     counts = gpu.train_accumulate_device(dev)
-    ref_counts = trainer.counts_from_encodes(imgs, w, h, chans)
+    ref_counts = ref_trainer.counts_from_encodes(imgs, w, h, chans)
     assert np.array_equal(counts, ref_counts)
     got = gpu.create_dynamic_block_prefix(counts, chans)
-    exp = trainer.create_prefix(ref_counts, chans)
+    exp = ref_trainer.create_prefix(ref_counts, chans)
     assert got[0] == exp[0] and got[1] == exp[1] and got[2] == exp[2]
     assert np.array_equal(got[4], exp[4])                       # code sizes
     used = exp[4] != 0
